@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- frames/sec of x-vector extraction (80-d fbank, 200-frame chunks, batches of 256) on N B200s.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
 
 One process per GPU (torchrun for N > 1).  A STEP is one pass of the hot path over one rank's shard of
 BASELINE.json configs[3]: 125 000 utterances (1 M over 8 GPUs) x 200 frames x 80-d, resident in HBM, through
@@ -33,6 +33,11 @@ round 1's measurement (one batch timed alone).
 `--impl reference` times that CPU port alone (the reference is Python/torch and cannot travel to the GPU box; the
 oracle restates it op for op, pinned by tests/golden) on a bounded sample of the same workload per step.
 XVB_BENCH_UTTS / XVB_BENCH_ECAPA_UTTS shrink the shards for smoke runs (the JSON line states the sizes used).
+
+--dump-outputs DIR writes what the timed path returned in its last step, after the timed region, as float32 .npy files:
+DIR/embeddings.npy holds the embedding table (native: the gathered (N x shard, 512) table; reference: the step's batch),
+cut to a fixed seeded sample of DUMP_ROWS rows when longer.  The inputs are seeded, so two builds run with the same
+arguments can be compared output for output; for that, N > 1 keeps equal shards (no balancing by measured speed).
 """
 import argparse
 import json
@@ -64,6 +69,7 @@ UTTS_PER_SPK = 100
 METRIC = "frames/sec x-vector extraction (80-d fbank)"
 UNIT = "frames/s"
 CPU_THREADS = 32                  # fixed thread count of the host arm (more threads than this slows ATen's small convs)
+DUMP_ROWS = 16384                 # --dump-outputs: at most this many embedding rows (32 MB of float32)
 
 
 def workload_config(world):
@@ -74,6 +80,16 @@ def workload_config(world):
             "l2_policy": "inputs larger than L2: %.1f GB of features per step per GPU, ~1.1 GB of activations per batch"
                          % (SHARD_UTTS * T * F * 4 / 1e9),
             "weights": "seeded synthetic checkpoint of the reference architecture"}
+
+
+def dump_outputs(dirname, **arrays):
+    """Each (rows, ...) tensor as DIR/<name>.npy in float32; longer than DUMP_ROWS rows: a fixed seeded sample of rows."""
+    os.makedirs(dirname, exist_ok=True)
+    for name, a in arrays.items():
+        if a.shape[0] > DUMP_ROWS:
+            rows = np.sort(np.random.default_rng(0).choice(a.shape[0], DUMP_ROWS, replace=False))
+            a = a[torch.from_numpy(rows).to(a.device)]
+        np.save(os.path.join(dirname, name + ".npy"), a.detach().float().cpu().numpy())
 
 
 def peaks():
@@ -224,8 +240,10 @@ def run_reference(args, rank, world):
             cpu_port_step(sd, x)
         t0 = time.perf_counter()
         for _ in range(args.steps):
-            cpu_port_step(sd, x)
+            out = cpu_port_step(sd, x)
         dt = time.perf_counter() - t0
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, embeddings=out.squeeze(2))
     value = args.steps * B * T / dt
     sample = ("each step = one whole 256 x 200 batch of the step's %d (a bounded sample of the same workload), batched "
               "forward of the oracle port, %d host threads" % ((SHARD_UTTS + B - 1) // B, threads))
@@ -653,7 +671,7 @@ def run_native(args, rank, world, local_rank):
     # GPUs of a box settle at different clocks (1447-1522 MHz in profiles/r04k) and a step ends when the slowest is done;
     # the reference balances its jobs the same way, by length (splitDataByLength.sh).  The total stays N x SHARD_UTTS.
     n_rank, row0, balance = [n] * world, rank * n, None
-    if table is not None and os.environ.get("XVB_BENCH_BALANCE", "1") != "0":
+    if table is not None and os.environ.get("XVB_BENCH_BALANCE", "1") != "0" and not args.dump_outputs:
         torch.cuda.synchronize()
         mine = statistics.mean(a.elapsed_time(b) for a, b in warm_ms[-2:])
         times = torch.zeros(world, dtype=torch.float64, device=dev)
@@ -697,6 +715,8 @@ def run_native(args, rank, world, local_rank):
     gather_ms = tm.max_over_ranks(statistics.median(ev[2 * i + 1].elapsed_time(ev[2 * i + 2]) for i in range(args.steps)))
     launches_per_step = ex.last_launches
     assert torch.isfinite(emb).all()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, embeddings=full)
     # the collective alone: inside a step its CUDA-event span also holds the wait for the slowest rank's shard
     gather_alone_ms, p2p_equals_nccl = 0.0, None
     if world > 1:
@@ -853,7 +873,11 @@ def main():
     ap.add_argument("--steps", type=int, default=10)
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="native", choices=["native", "reference"])
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step computed to DIR/<name>.npy (float32)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3)
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))

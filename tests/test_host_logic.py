@@ -316,6 +316,25 @@ def test_bench_shard_balancing_keeps_the_total_and_whole_batches():
     assert bench.balance_shards([1.0, 1.0], 2 * n, B, cap) == [125072, 124928]
 
 
+def test_bench_dump_outputs_writes_a_fixed_float32_sample_of_rows(tmp_path):
+    """bench.dump_outputs (--dump-outputs): float32 .npy files under 64 MB; a table longer than DUMP_ROWS is cut to the same
+    rows on every call, taken unchanged; a short one is written whole."""
+    import importlib.util
+    spec = importlib.util.spec_from_file_location("bench_mod", os.path.join(ROOT, "bench.py"))
+    bench = importlib.util.module_from_spec(spec)
+    spec.loader.exec_module(bench)
+    n = bench.DUMP_ROWS + 5000
+    table = torch.arange(n, dtype=torch.float64)[:, None].repeat(1, 512)      # row i holds i
+    for d in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / d), embeddings=table, short=table[:100])
+    a, b = np.load(tmp_path / "a" / "embeddings.npy"), np.load(tmp_path / "b" / "embeddings.npy")
+    assert a.dtype == np.float32 and a.shape == (bench.DUMP_ROWS, 512) and np.array_equal(a, b)
+    rows = a[:, 0]
+    assert np.all(a == rows[:, None]) and np.all(np.diff(rows) > 0) and rows[-1] < n
+    assert np.array_equal(np.load(tmp_path / "a" / "short.npy"), table[:100].float().numpy())
+    assert sum(os.path.getsize(p) for p in (tmp_path / "a").iterdir()) <= 64 << 20
+
+
 def test_bench_reference_arm_prints_the_contract_line():
     """`bench.py --impl reference` (the CPU arm the driver runs beside the native one): one JSON line with the contract's keys,
     `impl` = reference, the same metric / unit / config keys as the native arm, an `e2e` block without copies, no GPU needed;
