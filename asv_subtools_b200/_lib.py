@@ -20,7 +20,7 @@ class TdnnArgs(C.Structure):
                 ("y_hi", C.c_void_p), ("y_lo", C.c_void_p), ("ldy", C.c_int64),
                 ("y_f32", C.c_void_p), ("ldyf", C.c_int64),
                 ("B", C.c_int), ("T", C.c_int), ("Cin", C.c_int), ("Cout", C.c_int),
-                ("pool_partial", C.c_void_p), ("x_batch_stride", C.c_int64)]
+                ("pool_partial", C.c_void_p), ("x_batch_stride", C.c_int64), ("lengths", C.c_void_p)]
 MAX_TAPS = 16
 
 
@@ -113,6 +113,9 @@ SIGNATURES = {
     "xvb_extractor_wait": (_i, [_p, _i]),
     "xvb_extractor_extract_shard": (_i, [_p, _p, C.c_int64, _i, _i, _p, _p]),
     "xvb_extractor_extract_shard_host": (_i, [_p, _p, C.c_int64, _i, _i, _p, _p]),
+    "xvb_extractor_extract_ragged": (_i, [_p, _p, _p, _i, _p, _p]),
+    "xvb_extractor_extract_ragged_shard_host": (_i, [_p, _p, _p, _i64, _i, _i64, _p, _p]),
+    "xvb_ragged_plan": (_i, [_p, _i64, _i, _i64, _p, _p, _p]),
     "xvb_extractor_set_profiling": (_i, [_p, _i]),
     "xvb_extractor_kernel_times": (_i, [_p, C.POINTER(C.c_float), _i]),
     "xvb_extractor_last_launches": (_i, [_p]),

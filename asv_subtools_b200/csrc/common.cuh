@@ -103,6 +103,15 @@ int gemm_plan_build(GemmPlan** out, const xvb_tdnn_args_t& args, const TrialHist
 int gemm_plan_launch(const GemmPlan* plan, void* stream, float* y_f32_override = nullptr);
 void gemm_plan_destroy(GemmPlan* plan);
 
+// pooling.cu: launch of the fused-pooling merge behind xvb_pool_finalize; lengths (B, device) or NULL (all T frames)
+int pool_finalize_launch(const float* partial, int num_blocks, int frames_per_block, int B, int T, int C, float eps, int mode,
+                         const int32_t* lengths, float* out, uint16_t* out_hi, uint16_t* out_lo, int64_t ldo, void* stream);
+
+// core.cu: ragged (sum_T, C) fp32 frames, utterance b = rows offsets[b] .. offsets[b+1] (device int32), -> split planes
+// (B, pad_front + Tq + pad_back, ldp) with zero frames outside [0, L_b) of every utterance
+int split_ragged_frames(const float* x, const int32_t* offsets, int B, int Tq, int C, uint16_t* hi, uint16_t* lo, int64_t ldp,
+                        int pad_front, int pad_back, void* stream);
+
 // tdnn_gemm.cu: cuTensorMapEncodeTiled through the runtime's driver entry point (no -lcuda).
 int make_tensor_map(CUtensorMap* m, const void* base, int esize, int rank, const unsigned long long* dims,
                     const unsigned long long* strides_bytes, const unsigned* box, int swizzle_bytes);

@@ -118,6 +118,45 @@ __global__ void split_frames_kernel(const float* __restrict__ x, int B, int T, i
   }
 }
 
+// The same from a ragged batch: utterance b is rows offsets[b] .. offsets[b+1] of x (sum_T, C) and is
+// padded with zero frames up to Tq (so time steps [L_b, Tq) read as F.pad zeros, like the reference's
+// one-utterance extraction).
+__global__ void split_ragged_kernel(const float* __restrict__ x, const int32_t* __restrict__ offsets, int C,
+                                    __nv_bfloat16* __restrict__ hi, __nv_bfloat16* __restrict__ lo, long long ldp,
+                                    int pad_front, int Tp, long long total, int vec) {
+  const long long groups_per_row = ldp / 8;
+  for (long long i = blockIdx.x * (long long)blockDim.x + threadIdx.x; i < total; i += (long long)gridDim.x * blockDim.x) {
+    const long long r = i / groups_per_row;
+    const int c0 = (int)(i - r * groups_per_row) * 8;
+    const int b = (int)(r / Tp), t = (int)(r - (long long)b * Tp) - pad_front;
+    const int row0 = offsets[b], len = offsets[b + 1] - row0;
+    float v[8];
+#pragma unroll
+    for (int k = 0; k < 8; ++k) v[k] = 0.f;
+    if (t >= 0 && t < len) {
+      const float* src = x + ((long long)row0 + t) * C + c0;
+      if (vec && c0 + 8 <= C) {
+        const float4 a = *reinterpret_cast<const float4*>(src), c = *reinterpret_cast<const float4*>(src + 4);
+        v[0] = a.x; v[1] = a.y; v[2] = a.z; v[3] = a.w; v[4] = c.x; v[5] = c.y; v[6] = c.z; v[7] = c.w;
+      } else {
+#pragma unroll
+        for (int k = 0; k < 8; ++k) if (c0 + k < C) v[k] = src[k];
+      }
+    }
+    uint32_t h[4], l[4];
+#pragma unroll
+    for (int k = 0; k < 4; ++k) {
+      __nv_bfloat16 ah, al, bh, bl;
+      split_bf16(v[2 * k], ah, al);
+      split_bf16(v[2 * k + 1], bh, bl);
+      h[k] = pack_bf16x2(ah, bh);
+      l[k] = pack_bf16x2(al, bl);
+    }
+    *reinterpret_cast<uint4*>(hi + r * ldp + c0) = make_uint4(h[0], h[1], h[2], h[3]);
+    *reinterpret_cast<uint4*>(lo + r * ldp + c0) = make_uint4(l[0], l[1], l[2], l[3]);
+  }
+}
+
 // ------------------------------------------------------------------------------------------------
 // Reference weight (Cout, Cin, tot) -> packed K-major planes (Cout, ntaps*cin_p16), masked taps dropped.
 // ------------------------------------------------------------------------------------------------
@@ -174,6 +213,19 @@ static int grid_for(long long total, int block) {
   long long g = (total + block - 1) / block;
   const long long cap = (long long)sm_count() * 16;
   return (int)(g < 1 ? 1 : (g > cap ? cap : g));
+}
+
+int split_ragged_frames(const float* x, const int32_t* offsets, int B, int Tq, int C, uint16_t* hi, uint16_t* lo, int64_t ldp,
+                        int pad_front, int pad_back, void* stream) {
+  XVB_CHECK_ARG(x && offsets && hi && lo && B > 0 && Tq > 0 && C > 0 && ldp >= C && ldp % 8 == 0 && pad_front >= 0 && pad_back >= 0,
+                "split_ragged_frames: bad arguments");
+  const int Tp = pad_front + Tq + pad_back;
+  const long long total = (long long)B * Tp * (ldp / 8);
+  const int vec = (C % 4 == 0 && (uintptr_t)x % 16 == 0) ? 1 : 0;
+  split_ragged_kernel<<<grid_for(total, 256), 256, 0, (cudaStream_t)stream>>>(
+      x, offsets, C, reinterpret_cast<__nv_bfloat16*>(hi), reinterpret_cast<__nv_bfloat16*>(lo), ldp, pad_front, Tp, total, vec);
+  XVB_LAUNCH_CHECK();
+  return XVB_OK;
 }
 
 }  // namespace xvb

@@ -1,6 +1,6 @@
 // xvb-extract: Python-free x-vector extraction over the C ABI (SURVEY section 8f rank 4).
 //
-//   xvb-extract [--batch N] [--max-chunk N] [--cmn none|utt|sliding] [--cmn-window W] [--gpu-id ID]
+//   xvb-extract [--batch N] [--max-chunk N] [--ragged] [--cmn none|utt|sliding] [--cmn-window W] [--gpu-id ID]
 //               [--wav fbank|mfcc [--num-mel-bins N] [--num-ceps N] [--low-freq F] [--high-freq F]
 //                [--frame-length MS] [--frame-shift MS] [--energy-floor E] [--use-energy]]
 //               <model.xvbm> <feats-rspecifier | wav.scp> <vectors-wspecifier>
@@ -18,6 +18,9 @@
 //   * chunk rule of framework.py:34-47: T > max-chunk -> num_split = ceil(T/max), split = T/num_split,
 //     the last chunk takes the remainder, embedding = sum(len_i * emb_i) / T in fp32;
 //   * one "FV" vector per input key (order follows batch completion, which the wspecifier allows);
+//   * --ragged (TDNN x-vector models): instead of exact-length buckets, the chunks of a window of utterances (up to
+//     4 M frames) go through ONE xvb_extractor_extract_ragged_shard_host call -- length-sorted batches of mixed
+//     lengths, each chunk computed as if alone -- and the vectors are written in input order;
 //   * errors: message with "ERROR" on stderr, exit status 1 (the reference's shell greps for it,
 //     extract_xvectors_for_pytorch.sh:144-145).  No GPU / not a B200 -> error, there is no CPU path.
 #include <cuda_runtime.h>
@@ -61,6 +64,8 @@ struct Runner {
   xvb_ark_writer_t* out = nullptr;
   int F = 0, D = 0, batch = 256, cmn = 0, cmn_window = 300;
   float *d_feats = nullptr, *d_tmp = nullptr, *d_emb = nullptr, *h_feats = nullptr, *h_emb = nullptr;
+  float* h_ragged = nullptr;   // --ragged: a window's chunks back to back, pinned
+  size_t ragged_cap = 0;
   int32_t* d_off = nullptr;
   size_t cap_frames = 0;
   std::vector<Utt> utts;
@@ -90,22 +95,43 @@ struct Runner {
     if (ex) CK(xvb_extractor_extract(ex, d_feats, B, T, d_emb, nullptr), "xvb_extractor_extract");
     else CK(xvb_ecapa_extract(ec, d_feats, B, T, d_emb, nullptr), "xvb_ecapa_extract");
     CU(cudaMemcpy(h_emb, d_emb, (size_t)B * D * sizeof(float), cudaMemcpyDeviceToHost));
-    for (int i = 0; i < B; ++i) {
-      Utt& u = utts[items[i].utt];
-      const float len = (float)items[i].frames;
-      const float* e = h_emb + (size_t)i * D;
-      if (u.acc.empty()) u.acc.assign(D, 0.f);
-      for (int d = 0; d < D; ++d) u.acc[d] += len * e[d];
-      if (--u.pending == 0) {
-        const float total = (float)u.frames;
-        for (int d = 0; d < D; ++d) u.acc[d] /= total;
-        CK(xvb_ark_writer_put_vector(out, u.key.c_str(), u.acc.data(), D), "writing a vector");
-        std::vector<float>().swap(u.acc);
-        ++done_utts;
-        done_frames += u.frames;
-      }
-    }
+    for (int i = 0; i < B; ++i) accumulate(items[i], h_emb + (size_t)i * D);
     items.clear();
+  }
+
+  // --ragged: the window's chunks in one shard call; results come back in window order
+  void run_ragged(std::vector<Item>& items) {
+    if (items.empty()) return;
+    const int64_t n = (int64_t)items.size();
+    std::vector<int64_t> off((size_t)n + 1, 0);
+    for (int64_t i = 0; i < n; ++i) off[i + 1] = off[i] + items[i].frames;
+    if ((size_t)off[n] > ragged_cap) {
+      if (h_ragged) cudaFreeHost(h_ragged);
+      ragged_cap = (size_t)off[n] + (size_t)off[n] / 4;
+      CU(cudaMallocHost(&h_ragged, ragged_cap * F * sizeof(float)));
+    }
+    for (int64_t i = 0; i < n; ++i) memcpy(h_ragged + (size_t)off[i] * F, items[i].feats.data(), (size_t)items[i].frames * F * sizeof(float));
+    std::vector<float> emb((size_t)n * D);
+    CK(xvb_extractor_extract_ragged_shard_host(ex, h_ragged, off.data(), n, batch, 0, emb.data(), nullptr),
+       "xvb_extractor_extract_ragged_shard_host");
+    for (int64_t i = 0; i < n; ++i) accumulate(items[i], emb.data() + (size_t)i * D);
+    items.clear();
+  }
+
+  // chunk rule: sum(len_i * emb_i) / T, the vector is written when the utterance's last chunk is in
+  void accumulate(const Item& it, const float* e) {
+    Utt& u = utts[it.utt];
+    const float len = (float)it.frames;
+    if (u.acc.empty()) u.acc.assign(D, 0.f);
+    for (int d = 0; d < D; ++d) u.acc[d] += len * e[d];
+    if (--u.pending == 0) {
+      const float total = (float)u.frames;
+      for (int d = 0; d < D; ++d) u.acc[d] /= total;
+      CK(xvb_ark_writer_put_vector(out, u.key.c_str(), u.acc.data(), D), "writing a vector");
+      std::vector<float>().swap(u.acc);
+      ++done_utts;
+      done_frames += u.frames;
+    }
   }
 };
 
@@ -151,6 +177,7 @@ bool read_wav(const std::string& path, std::vector<float>* out, int* sample_rate
 int main(int argc, char** argv) {
   Runner r;
   int max_chunk = 10000, gpu = 0;
+  bool ragged = false;
   std::string wav_type;
   xvb_fbank_opts_t fo;
   xvb_fbank_default_opts(&fo);
@@ -163,6 +190,7 @@ int main(int argc, char** argv) {
       return argv[++i];
     };
     if (a == "--batch") r.batch = atoi(val("--batch"));
+    else if (a == "--ragged") ragged = true;
     else if (a == "--max-chunk") max_chunk = atoi(val("--max-chunk"));
     else if (a == "--cmn-window") r.cmn_window = atoi(val("--cmn-window"));
     else if (a == "--gpu-id") gpu = atoi(val("--gpu-id"));
@@ -180,7 +208,7 @@ int main(int argc, char** argv) {
       r.cmn = m == "none" ? 0 : m == "utt" ? 1 : m == "sliding" ? 2 : -1;
       if (r.cmn < 0) { fprintf(stderr, "ERROR: xvb-extract: --cmn must be none, utt or sliding\n"); return 1; }
     } else if (a == "--help" || a == "-h") {
-      printf("usage: xvb-extract [--batch N] [--max-chunk N] [--cmn none|utt|sliding] [--cmn-window W] [--gpu-id ID]\n"
+      printf("usage: xvb-extract [--batch N] [--max-chunk N] [--ragged] [--cmn none|utt|sliding] [--cmn-window W] [--gpu-id ID]\n"
              "                   [--wav fbank|mfcc [--num-mel-bins N] [--num-ceps N] [--low-freq F] [--high-freq F]\n"
              "                    [--frame-length MS] [--frame-shift MS] [--energy-floor E] [--use-energy]]\n"
              "                   <model.xvbm> <feats-rspecifier | wav.scp> <vectors-wspecifier>\n");
@@ -205,6 +233,7 @@ int main(int argc, char** argv) {
     if (!mf || fread(magic, 1, 8, mf) != 8) { fprintf(stderr, "ERROR: xvb-extract: cannot read model file '%s'\n", pos[0]); return 1; }
     fclose(mf);
     if (memcmp(magic, "XVBE0001", 8) == 0) {
+      if (ragged) { fprintf(stderr, "ERROR: xvb-extract: --ragged needs a TDNN x-vector model; ECAPA-TDNN has no ragged path yet (drop --ragged)\n"); return 1; }
       CK(xvb_ecapa_load(&r.ec, pos[0]), "loading the ECAPA model");
       r.F = xvb_ecapa_feat_dim(r.ec);
       r.D = xvb_ecapa_embed_dim(r.ec);
@@ -273,6 +302,9 @@ int main(int argc, char** argv) {
   const bool to_stdout = wspec == "-" || (wspec.size() >= 2 && wspec.compare(wspec.size() - 2, 2, ":-") == 0);   // keep the ark stream clean
   std::map<int, std::vector<Item>> buckets;   // frames -> pending chunks of that length
   size_t pending = 0;
+  std::vector<Item> window;                   // --ragged: chunks in input order
+  size_t window_frames = 0;
+  const size_t max_window_frames = 4000000;
   const size_t max_pending = (size_t)r.batch * 64;
   const char* key;
   int rows, cols, rc;
@@ -305,10 +337,19 @@ int main(int argc, char** argv) {
       it.frames = len;
       it.feats.assign(data + (size_t)off * cols, data + (size_t)(off + len) * cols);
       off += len;
+      if (ragged) {
+        window.push_back(std::move(it));
+        window_frames += len;
+        continue;
+      }
       std::vector<Item>& b = buckets[len];
       b.push_back(std::move(it));
       ++pending;
       if ((int)b.size() == r.batch) { pending -= b.size(); r.run(b); }
+    }
+    if (window_frames >= max_window_frames) {
+      r.run_ragged(window);
+      window_frames = 0;
     }
     if (pending > max_pending) {   // bound host memory: flush the fullest bucket
       auto best = buckets.begin();
@@ -320,6 +361,7 @@ int main(int argc, char** argv) {
   }
   if (rc < 0) die("reading features");
   for (auto& kv : buckets) r.run(kv.second);
+  r.run_ragged(window);
   if (in) xvb_ark_reader_close(in);
   if (wav_scp) fclose(wav_scp);
   if (fb) xvb_fbank_destroy(fb);

@@ -5,8 +5,12 @@
 // reference's C++ runtime (runtime/bin/extractor_main.cc, runtime/speaker/torch_asv_model.cc).
 #include <cuda_runtime.h>
 #include <stdlib.h>
+#include <string.h>
 
+#include <algorithm>
 #include <map>
+#include <numeric>
+#include <tuple>
 #include <utility>
 #include <vector>
 
@@ -84,11 +88,33 @@ struct xvb_extractor {
   int pad_front = 0, pad_back = 0;
   float* pool_partial = nullptr;
   size_t pool_partial_cap = 0;
-  // launch plans per batch shape; they hold pointers into the workspace, so anything that reallocates it clears them
-  std::map<std::pair<int, int>, StepPlan*> plans;
+  // ragged batches: [offsets (B+1) | lengths (B)] of the current batch on the device (2 * cap_B + 1 int32, part of the
+  // workspace), its pinned host staging and the event that tells when the last upload has left the staging buffer
+  int32_t* ragged_meta = nullptr;
+  int32_t* ragged_meta_host = nullptr;
+  size_t ragged_meta_host_cap = 0;
+  cudaEvent_t ev_meta = nullptr;
+  float* ragged_emb_host = nullptr;          // shard call: embeddings in batch (length-sorted) order, pinned
+  size_t ragged_emb_host_cap = 0;
+  int32_t* shard_meta = nullptr;             // shard call: every batch's [offsets | lengths] block
+  size_t shard_meta_cap = 0;
+  // launch plans per batch shape (B, T, ragged); they hold pointers into the workspace, so anything that reallocates it
+  // clears them.  Every plan owns split-K scratch, and a stream of ragged batches can visit many padded lengths, so
+  // the ragged plans are dropped together once there are kMaxRaggedPlans of them.
+  static constexpr int kMaxRaggedPlans = 64;
+  std::map<std::tuple<int, int, bool>, StepPlan*> plans;
+  int ragged_plans = 0;
   void drop_plans() {
     for (auto& kv : plans) delete kv.second;
     plans.clear();
+    ragged_plans = 0;
+  }
+  void drop_ragged_plans() {
+    for (auto it = plans.begin(); it != plans.end();) {
+      if (std::get<2>(it->first)) { delete it->second; it = plans.erase(it); }
+      else ++it;
+    }
+    ragged_plans = 0;
   }
   // Two-lane shard pipeline: batches of a shard alternate between this extractor and `lane1`, a shallow twin that
   // shares the packed weights but owns its workspace and plans, each on its own stream.  The tcgen05 layer kernels
@@ -124,8 +150,8 @@ struct xvb_extractor {
     drop_plans();
     cudaFree(in_hi); cudaFree(in_lo);
     for (int i = 0; i < 2; ++i) { cudaFree(act_hi[i]); cudaFree(act_lo[i]); cudaFree(seg_hi[i]); cudaFree(seg_lo[i]); }
-    cudaFree(last_f32); cudaFree(stats); cudaFree(stats_hi); cudaFree(stats_lo); cudaFree(emb_ws);
-    in_hi = in_lo = nullptr; last_f32 = stats = emb_ws = nullptr; stats_hi = stats_lo = nullptr;
+    cudaFree(last_f32); cudaFree(stats); cudaFree(stats_hi); cudaFree(stats_lo); cudaFree(emb_ws); cudaFree(ragged_meta);
+    in_hi = in_lo = nullptr; last_f32 = stats = emb_ws = nullptr; stats_hi = stats_lo = nullptr; ragged_meta = nullptr;
     for (int i = 0; i < 2; ++i) act_hi[i] = act_lo[i] = seg_hi[i] = seg_lo[i] = nullptr;
     cap_frames = 0; cap_B = 0;
   }
@@ -263,13 +289,15 @@ static int reserve(xvb_extractor* h, int B, int T) {
       if ((rc = dev_alloc(&h->seg_hi[i], (size_t)nb * h->max_seg_c))) return rc;
       if ((rc = dev_alloc(&h->seg_lo[i], (size_t)nb * h->max_seg_c))) return rc;
     }
+  if ((rc = dev_alloc(&h->ragged_meta, (size_t)2 * nb + 1))) return rc;
   h->cap_frames = nf;
   h->cap_B = nb;
   return XVB_OK;
 }
 
-// Build the launch plan of one batch shape (see StepPlan).  On failure nothing is cached.
-static int build_step_plan(xvb_extractor* h, int B, int T, StepPlan** out) {
+// Build the launch plan of one batch shape (see StepPlan).  On failure nothing is cached.  A ragged plan's frame layers
+// mask with the lengths of the batch's [offsets | lengths] block in h->ragged_meta.
+static int build_step_plan(xvb_extractor* h, int B, int T, bool ragged, StepPlan** out) {
   StepPlan* sp = new StepPlan();
   struct Guard { StepPlan* p; ~Guard() { delete p; } } guard{sp};
   int rc;
@@ -301,6 +329,7 @@ static int build_step_plan(xvb_extractor* h, int B, int T, StepPlan** out) {
     a.context_host = L.ctx; a.ntaps = L.ntaps;
     a.y_hi = y_hi; a.y_lo = y_lo; a.ldy = L.Cout;
     a.B = B; a.T = T; a.Cin = L.Cin; a.Cout = L.Cout;
+    if (ragged) a.lengths = h->ragged_meta + B + 1;
     const int ctx0 = 0;
     if (i == 0 && h->im2col_first) {   // window of ntaps consecutive frames = one long row of the padded planes
       a.context_host = &ctx0; a.ntaps = 1; a.Cin = L.ntaps * L.Cin;
@@ -338,9 +367,9 @@ static int build_step_plan(xvb_extractor* h, int B, int T, StepPlan** out) {
   return XVB_OK;
 }
 
-extern "C" int xvb_extractor_extract(xvb_extractor_t* h, const float* feats, int B, int T, float* emb, void* stream) {
-  XVB_CHECK_ARG(h && h->finalized, "xvb_extractor_extract: extractor not finalized");
-  XVB_CHECK_ARG(feats && emb && B > 0 && T > 0, "xvb_extractor_extract: bad arguments");
+// The whole stack for one batch.  Equal lengths: feats (B, T, F).  Ragged (`ragged`): feats (sum_T, F) laid out by the
+// offsets already in h->ragged_meta, T = the padded length Tq.
+static int run_stack(xvb_extractor* h, const float* feats, int B, int T, bool ragged, float* emb, void* stream) {
   int rc = reserve(h, B, T);
   if (rc) return rc;
   const long before = g_launches;
@@ -348,7 +377,8 @@ extern "C" int xvb_extractor_extract(xvb_extractor_t* h, const float* feats, int
   if (!h->in_shard) h->events_used = 0;   // a shard call keeps the events of all its batches
   h->events_stream = cs;
   StepPlan* sp = nullptr;
-  auto it = h->plans.find(std::make_pair(B, T));
+  const auto key = std::make_tuple(B, T, ragged);
+  auto it = h->plans.find(key);
   if (it != h->plans.end()) {
     sp = it->second;
   } else {
@@ -363,20 +393,25 @@ extern "C" int xvb_extractor_extract(xvb_extractor_t* h, const float* feats, int
         h->pool_partial_cap = need;
       }
     }
-    rc = build_step_plan(h, B, T, &sp);
+    if (ragged && h->ragged_plans >= xvb_extractor::kMaxRaggedPlans) h->drop_ragged_plans();
+    rc = build_step_plan(h, B, T, ragged, &sp);
     if (rc == -1000) {        // the driver refused the overlapping (im2col) tensor map: plain first layer from now on
       h->im2col_first = false;
       h->pad_front = h->pad_back = 0;
       h->drop_plans();
-      return xvb_extractor_extract(h, feats, B, T, emb, stream);
+      return run_stack(h, feats, B, T, ragged, emb, stream);
     }
     if (rc) return rc;
-    h->plans[std::make_pair(B, T)] = sp;
+    h->plans[key] = sp;
+    if (ragged) ++h->ragged_plans;
   }
   if ((rc = h->mark(cs))) return rc;
   // 1. stage the frame matrix as split planes (framework.py:28-33 staging); for the im2col first layer with
   //    the zero frames of F.pad (components.py:117) written out around every utterance
-  if (h->im2col_first)
+  if (ragged)   // zero frames from L_b on: what the reference's per-utterance F.pad reads past the end
+    rc = split_ragged_frames(feats, h->ragged_meta, B, T, h->feat_dim, h->in_hi, h->in_lo, h->ldf, h->pad_front, h->pad_back,
+                             stream);
+  else if (h->im2col_first)
     rc = xvb_split_frames(feats, B, T, h->feat_dim, h->in_hi, h->in_lo, h->ldf, h->pad_front, h->pad_back, stream);
   else
     rc = xvb_split_f32(feats, (int64_t)B * T, h->feat_dim, h->feat_dim, h->in_hi, h->in_lo, h->ldf, stream);
@@ -389,9 +424,9 @@ extern "C" int xvb_extractor_extract(xvb_extractor_t* h, const float* feats, int
   }
   // 3. statistics pooling (xvector.py:90, pooling.py:58-67)
   const int cl = h->frame.back().Cout;
-  if (h->fused_pooling)
-    rc = xvb_pool_finalize(h->pool_partial, sp->pool_blocks, sp->pool_tb, B, T, cl, h->pooling_eps, 0, h->stats, h->stats_hi,
-                           h->stats_lo, 2 * cl, stream);
+  if (h->fused_pooling)   // ragged: mean and std over each utterance's own L_b frames
+    rc = pool_finalize_launch(h->pool_partial, sp->pool_blocks, sp->pool_tb, B, T, cl, h->pooling_eps, 0,
+                              ragged ? h->ragged_meta + B + 1 : nullptr, h->stats, h->stats_hi, h->stats_lo, 2 * cl, stream);
   else
     rc = xvb_stats_pool(h->last_f32, cl, B, T, cl, h->pooling_eps, h->stats, h->stats_hi, h->stats_lo, 2 * cl, stream);
   if (rc) return rc;
@@ -403,6 +438,82 @@ extern "C" int xvb_extractor_extract(xvb_extractor_t* h, const float* feats, int
     if ((rc = h->mark(cs))) return rc;
   }
   h->last_launches = (int)(g_launches - before);
+  return XVB_OK;
+}
+
+extern "C" int xvb_extractor_extract(xvb_extractor_t* h, const float* feats, int B, int T, float* emb, void* stream) {
+  XVB_CHECK_ARG(h && h->finalized, "xvb_extractor_extract: extractor not finalized");
+  XVB_CHECK_ARG(feats && emb && B > 0 && T > 0, "xvb_extractor_extract: bad arguments");
+  return run_stack(h, feats, B, T, false, emb, stream);
+}
+
+static constexpr int kRaggedQuantum = 32;                 // padded length Tq = round_up(max L_b, 32)
+static constexpr int64_t kRaggedDefaultMaxFrames = 262144;  // 256 utterances x 1024 frames
+
+// The ragged path needs the fused pooling epilogue (the only pooling that counts per-utterance lengths) and writes no
+// replicated table.
+static int ragged_state_ok(const xvb_extractor* h, const char* fn) {
+  if (!h->fused_pooling) { set_error("%s: needs fused pooling (xvb_extractor_set_fused_pooling(h, 1))", fn); return XVB_ESTATE; }
+  if (h->gather_n) { set_error("%s: a gather table is set; ragged batches do not write replicated tables", fn); return XVB_ESTATE; }
+  return XVB_OK;
+}
+
+extern "C" int xvb_extractor_extract_ragged(xvb_extractor_t* h, const float* feats, const int32_t* offsets_host, int B, float* emb,
+                                            void* stream) {
+  XVB_CHECK_ARG(h && h->finalized, "xvb_extractor_extract_ragged: extractor not finalized");
+  XVB_CHECK_ARG(feats && offsets_host && emb && B > 0 && offsets_host[0] >= 0, "xvb_extractor_extract_ragged: bad arguments");
+  int rc = ragged_state_ok(h, "xvb_extractor_extract_ragged");
+  if (rc) return rc;
+  int max_len = 0;
+  for (int b = 0; b < B; ++b) {
+    const int len = offsets_host[b + 1] - offsets_host[b];
+    XVB_CHECK_ARG(offsets_host[b + 1] > offsets_host[b], "xvb_extractor_extract_ragged: utterance %d has %d frames (need >= 1)", b, len);
+    max_len = len > max_len ? len : max_len;
+  }
+  XVB_CHECK_ARG(max_len <= (1 << 30), "xvb_extractor_extract_ragged: utterance too long");
+  const int Tq = (int)round_up(max_len, kRaggedQuantum);
+  if ((rc = reserve(h, B, Tq))) return rc;   // before the upload: it may reallocate ragged_meta
+  cudaStream_t s = (cudaStream_t)stream;
+  const size_t n = (size_t)2 * B + 1;
+  if (!h->ev_meta) XVB_CUDA(cudaEventCreateWithFlags(&h->ev_meta, cudaEventDisableTiming));
+  XVB_CUDA(cudaEventSynchronize(h->ev_meta));   // the previous upload has left the pinned staging buffer
+  if (n > h->ragged_meta_host_cap) {
+    cudaFreeHost(h->ragged_meta_host);
+    h->ragged_meta_host = nullptr; h->ragged_meta_host_cap = 0;
+    XVB_CUDA(cudaMallocHost((void**)&h->ragged_meta_host, n * sizeof(int32_t)));
+    h->ragged_meta_host_cap = n;
+  }
+  for (int b = 0; b <= B; ++b) h->ragged_meta_host[b] = offsets_host[b];
+  for (int b = 0; b < B; ++b) h->ragged_meta_host[B + 1 + b] = offsets_host[b + 1] - offsets_host[b];
+  // on the launching stream: the kernels of an earlier batch on it have read the old block before this overwrites it
+  XVB_CUDA(cudaMemcpyAsync(h->ragged_meta, h->ragged_meta_host, n * sizeof(int32_t), cudaMemcpyHostToDevice, s));
+  XVB_CUDA(cudaEventRecord(h->ev_meta, s));
+  return run_stack(h, feats, B, Tq, true, emb, stream);
+}
+
+extern "C" int xvb_ragged_plan(const int64_t* offsets_host, int64_t N, int batch, int64_t max_frames, int32_t* order_out,
+                               int64_t* batch_first_out, int64_t* num_batches_out) {
+  XVB_CHECK_ARG(offsets_host && order_out && batch_first_out && num_batches_out && N > 0 && N <= INT32_MAX && batch > 0 &&
+                offsets_host[0] >= 0, "xvb_ragged_plan: bad arguments");
+  if (max_frames <= 0) max_frames = kRaggedDefaultMaxFrames;
+  for (int64_t i = 0; i < N; ++i) {
+    const int64_t len = offsets_host[i + 1] - offsets_host[i];
+    XVB_CHECK_ARG(len >= 1 && len <= (1 << 30), "xvb_ragged_plan: utterance %lld has %lld frames (need 1 .. 2^30)", (long long)i,
+                  (long long)len);
+  }
+  auto len = [&](int32_t i) { return offsets_host[i + 1] - offsets_host[i]; };
+  std::iota(order_out, order_out + N, 0);
+  std::stable_sort(order_out, order_out + N, [&](int32_t a, int32_t b) { return len(a) < len(b); });
+  // ascending lengths: the utterance that joins a batch sets its padded length
+  int64_t nb = 0;
+  for (int64_t i = 0; i < N;) {
+    batch_first_out[nb++] = i;
+    int64_t j = i + 1;
+    while (j < N && j - i < batch && (j - i + 1) * round_up(len(order_out[j]), kRaggedQuantum) <= max_frames) ++j;
+    i = j;
+  }
+  batch_first_out[nb] = N;
+  *num_batches_out = nb;
   return XVB_OK;
 }
 
@@ -628,6 +739,106 @@ extern "C" int xvb_extractor_extract_shard_host(xvb_extractor_t* h, const float*
   return XVB_OK;
 }
 
+// A shard of N utterances of any lengths through host buffers: xvb_ragged_plan's batches (length-sorted) through the same
+// two-lane / four-slot pipeline as xvb_extractor_extract_shard_host.  A batch's utterances are gathered into its device
+// slot with one copy per run of consecutive input utterances; its [offsets | lengths] block, uploaded for all batches at
+// the start, is copied into the lane's workspace on the lane's stream.  Embeddings come back in batch order and are put
+// into input order on the host after the final synchronisation.
+extern "C" int xvb_extractor_extract_ragged_shard_host(xvb_extractor_t* h, const float* feats_host, const int64_t* offsets_host,
+                                                       int64_t N, int batch, int64_t max_frames, float* emb_host, void* stream) {
+  XVB_CHECK_ARG(h && h->finalized && feats_host && offsets_host && emb_host && N > 0 && batch > 0,
+                "xvb_extractor_extract_ragged_shard_host: bad arguments");
+  XVB_CHECK_ARG(!h->slot_busy[0] && !h->slot_busy[1], "xvb_extractor_extract_ragged_shard_host: a submit_host slot is still in flight");
+  int rc = ragged_state_ok(h, "xvb_extractor_extract_ragged_shard_host");
+  if (rc) return rc;
+  std::vector<int32_t> order((size_t)N);
+  std::vector<int64_t> first((size_t)N + 1);
+  int64_t nbatch = 0;
+  if ((rc = xvb_ragged_plan(offsets_host, N, batch, max_frames, order.data(), first.data(), &nbatch))) return rc;
+  const int F = h->feat_dim, D = h->segment.back().Cout;
+  // every batch's [offsets (b+1) | lengths (b)] block, offsets relative to the batch's packed features
+  std::vector<int32_t> meta;
+  meta.reserve((size_t)(2 * N + nbatch));
+  std::vector<size_t> meta_at((size_t)nbatch);
+  int64_t max_rows = 0, bmax = 0;
+  for (int64_t k = 0; k < nbatch; ++k) {
+    const int64_t i0 = first[k], i1 = first[k + 1];
+    meta_at[k] = meta.size();
+    int64_t rows = 0;
+    meta.push_back(0);
+    for (int64_t i = i0; i < i1; ++i) {
+      rows += offsets_host[order[i] + 1] - offsets_host[order[i]];
+      XVB_CHECK_ARG(rows <= INT32_MAX, "xvb_extractor_extract_ragged_shard_host: a batch exceeds 2^31 frames");
+      meta.push_back((int32_t)rows);
+    }
+    for (int64_t i = i0; i < i1; ++i) meta.push_back((int32_t)(offsets_host[order[i] + 1] - offsets_host[order[i]]));
+    max_rows = std::max(max_rows, rows);
+    bmax = std::max(bmax, i1 - i0);
+  }
+  cudaStream_t s = (cudaStream_t)stream;
+  if ((rc = ensure_pipeline(h))) return rc;
+  constexpr int S = xvb_extractor::kSlots;
+  for (int slot = 0; slot < S; ++slot)
+    if ((rc = reserve_slot(h, slot, (size_t)max_rows * F, (size_t)bmax * D))) return rc;
+  if (meta.size() > h->shard_meta_cap) {
+    cudaFree(h->shard_meta);
+    h->shard_meta = nullptr; h->shard_meta_cap = 0;
+    if ((rc = dev_alloc(&h->shard_meta, meta.size()))) return rc;
+    h->shard_meta_cap = meta.size();
+  }
+  const size_t ne = (size_t)N * D;
+  if (ne > h->ragged_emb_host_cap) {
+    cudaFreeHost(h->ragged_emb_host);
+    h->ragged_emb_host = nullptr; h->ragged_emb_host_cap = 0;
+    XVB_CUDA(cudaMallocHost((void**)&h->ragged_emb_host, ne * sizeof(float)));
+    h->ragged_emb_host_cap = ne;
+  }
+  // `meta` outlives the copy: this call returns only after synchronising `stream`
+  XVB_CUDA(cudaMemcpyAsync(h->shard_meta, meta.data(), meta.size() * sizeof(int32_t), cudaMemcpyHostToDevice, s));
+  const bool lanes = lanes_enabled() && !h->profiling && nbatch > 1;
+  if (lanes) {
+    if ((rc = ensure_lanes(h))) return rc;
+    if ((rc = lanes_fork(h, s))) return rc;
+  }
+  int launches = 0;
+  for (int64_t k = 0; k < nbatch; ++k) {
+    const int64_t i0 = first[k];
+    const int b = (int)(first[k + 1] - i0);
+    const int max_len = meta[meta_at[k] + b + 1 + b - 1];   // the batch is sorted by length: the last one is the longest
+    const int Tq = (int)round_up(max_len, kRaggedQuantum);
+    const int slot = (int)(k % S);
+    xvb_extractor* lane = (lanes && (k & 1)) ? h->lane1 : h;
+    cudaStream_t ls = lanes ? h->lane_stream[k & 1] : s;
+    if (k >= S) XVB_CUDA(cudaStreamWaitEvent(h->copy_stream, h->ev_done[slot], 0));   // batch k-4 has left this slot
+    float* dst = h->p_feats[slot];
+    for (int64_t i = i0; i < i0 + b;) {   // runs of consecutive input utterances are contiguous in feats_host
+      int64_t j = i + 1;
+      while (j < i0 + b && order[j] == order[j - 1] + 1) ++j;
+      const int64_t r0 = offsets_host[order[i]], r1 = offsets_host[order[j - 1] + 1];
+      XVB_CUDA(cudaMemcpyAsync(dst, feats_host + (size_t)r0 * F, (size_t)(r1 - r0) * F * sizeof(float), cudaMemcpyHostToDevice,
+                               h->copy_stream));
+      dst += (size_t)(r1 - r0) * F;
+      i = j;
+    }
+    XVB_CUDA(cudaEventRecord(h->ev_h2d[slot], h->copy_stream));
+    XVB_CUDA(cudaStreamWaitEvent(ls, h->ev_h2d[slot], 0));
+    if ((rc = reserve(lane, b, Tq))) return rc;
+    XVB_CUDA(cudaMemcpyAsync(lane->ragged_meta, h->shard_meta + meta_at[k], (size_t)(2 * b + 1) * sizeof(int32_t),
+                             cudaMemcpyDeviceToDevice, ls));
+    if ((rc = run_stack(lane, h->p_feats[slot], b, Tq, true, h->p_emb[slot], ls))) return rc;
+    XVB_CUDA(cudaMemcpyAsync(h->ragged_emb_host + (size_t)i0 * D, h->p_emb[slot], (size_t)b * D * sizeof(float),
+                             cudaMemcpyDeviceToHost, ls));
+    XVB_CUDA(cudaEventRecord(h->ev_done[slot], ls));
+    launches += lane->last_launches;
+  }
+  if (lanes && (rc = lanes_join(h, s))) return rc;
+  XVB_CUDA(cudaStreamSynchronize(s));
+  for (int64_t i = 0; i < N; ++i)
+    memcpy(emb_host + (size_t)order[i] * D, h->ragged_emb_host + (size_t)i * D, (size_t)D * sizeof(float));
+  h->last_launches = launches;
+  return XVB_OK;
+}
+
 extern "C" int xvb_extractor_set_fused_pooling(xvb_extractor_t* h, int enable) {
   XVB_CHECK_ARG(h, "xvb_extractor_set_fused_pooling: null extractor");
   if (h->fused_pooling != (enable != 0)) h->drop_plans();
@@ -676,6 +887,8 @@ extern "C" void xvb_extractor_destroy(xvb_extractor_t* h) {
     if (h->ev_done[i]) cudaEventDestroy(h->ev_done[i]);
   }
   if (h->copy_stream) cudaStreamDestroy(h->copy_stream);
+  if (h->ev_meta) cudaEventDestroy(h->ev_meta);
+  cudaFreeHost(h->ragged_meta_host); cudaFreeHost(h->ragged_emb_host); cudaFree(h->shard_meta);
   cudaFree(h->h_feats); cudaFree(h->h_emb); cudaFree(h->pool_partial);
   if (!h->is_lane)
     for (auto* v : {&h->frame, &h->segment})

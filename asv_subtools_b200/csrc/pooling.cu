@@ -142,13 +142,19 @@ stats_pool_tma_kernel(const __grid_constant__ CUtensorMap map_x, int T, int C, f
 }
 
 // Merge the per-time-block [mean | M2] partials written by the fused GEMM epilogue (Chan's update,
-// block k has n_k = min(Tb, T - k*Tb) frames), then apply the reference's std definition.
+// block k has n_k = min(Tb, T - k*Tb) frames), then apply the reference's std definition.  Ragged batch
+// (lengths != NULL): utterance b has L = lengths[b] frames, so only its first ceil(L / Tb) blocks were
+// written -- the rest are never read -- and L is the divisor.
 __global__ void pool_finalize_kernel(const float* __restrict__ partial, int nblk, int Tb, int B, int T, int C, float eps,
-                                     int mode, float* __restrict__ out, __nv_bfloat16* __restrict__ out_hi,
-                                     __nv_bfloat16* __restrict__ out_lo, long long ldo) {
+                                     int mode, const int* __restrict__ lengths, float* __restrict__ out,
+                                     __nv_bfloat16* __restrict__ out_hi, __nv_bfloat16* __restrict__ out_lo, long long ldo) {
   const int c = (blockIdx.x * blockDim.x + threadIdx.x) * 4;
   const int b = blockIdx.y;
   if (c >= C) return;
+  if (lengths) {
+    T = min(lengths[b], T);
+    nblk = min(nblk, (T + Tb - 1) / Tb);
+  }
   float n = 0.f;
   float mean[4] = {0.f, 0.f, 0.f, 0.f}, m2[4] = {0.f, 0.f, 0.f, 0.f};
   for (int k = 0; k < nblk; ++k) {
@@ -185,6 +191,16 @@ __global__ void pool_finalize_kernel(const float* __restrict__ partial, int nblk
   }
 }
 
+int pool_finalize_launch(const float* partial, int num_blocks, int frames_per_block, int B, int T, int C, float eps, int mode,
+                         const int32_t* lengths, float* out, uint16_t* out_hi, uint16_t* out_lo, int64_t ldo, void* stream) {
+  dim3 grid((C / 4 + 127) / 128, B);
+  pool_finalize_kernel<<<grid, 128, 0, (cudaStream_t)stream>>>(partial, num_blocks, frames_per_block, B, T, C, eps, mode, lengths,
+                                                              out, reinterpret_cast<__nv_bfloat16*>(out_hi),
+                                                              reinterpret_cast<__nv_bfloat16*>(out_lo), ldo);
+  XVB_LAUNCH_CHECK();
+  return XVB_OK;
+}
+
 }  // namespace xvb
 
 using namespace xvb;
@@ -200,12 +216,7 @@ extern "C" int xvb_pool_finalize(const float* partial, int num_blocks, int frame
   XVB_CHECK_ARG((out_hi != nullptr) == (out_lo != nullptr), "xvb_pool_finalize: out_hi/out_lo must both be set or both NULL");
   if (out_hi) XVB_CHECK_ARG(ldo >= 2 * C && ldo % 4 == 0, "xvb_pool_finalize: ldo too small / unaligned");
   XVB_CHECK_ARG(mode == 0 || mode == 1, "xvb_pool_finalize: mode must be 0 or 1");
-  dim3 grid((C / 4 + 127) / 128, B);
-  pool_finalize_kernel<<<grid, 128, 0, (cudaStream_t)stream>>>(partial, num_blocks, frames_per_block, B, T, C, eps, mode, out,
-                                                              reinterpret_cast<__nv_bfloat16*>(out_hi),
-                                                              reinterpret_cast<__nv_bfloat16*>(out_lo), ldo);
-  XVB_LAUNCH_CHECK();
-  return XVB_OK;
+  return pool_finalize_launch(partial, num_blocks, frames_per_block, B, T, C, eps, mode, nullptr, out, out_hi, out_lo, ldo, stream);
 }
 
 extern "C" int xvb_stats_pool(const float* x, int64_t ldx, int B, int T, int C, float eps, float* out, uint16_t* out_hi,

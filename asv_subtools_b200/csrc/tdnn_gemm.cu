@@ -91,6 +91,7 @@ struct TdnnGemmParams {
   long long ldy;
   float* y_f32;
   long long ldyf;
+  const int* lengths;     // ragged batch (kMask only): valid frames per utterance, device
 };
 
 // kCta = 1: one CTA per 128 x BLOCK_N tile.  kCta = 2: a CTA pair (cluster of 2, tcgen05
@@ -146,7 +147,9 @@ __device__ __forceinline__ bool decode_tile(const TdnnGemmParams& p, int tile, i
 }
 
 // kHist: the epilogue bins the scores into a trial histogram instead of storing them (scoring.cu).
-template <int BLOCK_N, int kCta, int kNSub, bool kPool, bool kHist>
+// kMask: ragged batch -- rows t >= lengths[b] store exact zeros (the F.pad zeros the next layer's taps must read) and the
+// pooling epilogue counts lengths[b] frames.  A separate instantiation, so the equal-length kernels are untouched.
+template <int BLOCK_N, int kCta, int kNSub, bool kPool, bool kHist, bool kMask>
 __global__ void __launch_bounds__(kNumThreads, 1)
 tdnn_gemm_bf16x3_kernel(const __grid_constant__ CUtensorMap map_a_hi, const __grid_constant__ CUtensorMap map_a_lo,
                         const __grid_constant__ CUtensorMap map_a2_hi, const __grid_constant__ CUtensorMap map_a2_lo,
@@ -399,7 +402,12 @@ tdnn_gemm_bf16x3_kernel(const __grid_constant__ CUtensorMap map_a_hi, const __gr
         auto group = [&](const float* x, int col0, auto gtag) {
           constexpr int G = decltype(gtag)::value;
           const int tt0 = col0 & (p.Tb - 1);
-          int nv = p.T - (th0 + tt0);                              // valid frames of this group (warp-uniform)
+          int len = p.T;
+          if constexpr (kMask) {                                   // the group's frames belong to one utterance
+            const int bb = bh0 + (col0 >> p.log2_tb);
+            len = bb < p.B ? __ldg(p.lengths + bb) : 0;
+          }
+          int nv = len - (th0 + tt0);                              // valid frames of this group (warp-uniform)
           nv = nv < 0 ? 0 : (nv > G ? G : nv);
           float sum = 0.f;
 #pragma unroll
@@ -463,6 +471,8 @@ tdnn_gemm_bf16x3_kernel(const __grid_constant__ CUtensorMap map_a_hi, const __gr
         else mbar_arrive_cluster(&tmem_empty_bar[acc], 0);
         continue;
       }
+      bool masked = false;                                 // frame past the end of its utterance: store zeros
+      if constexpr (kMask) masked = valid && t >= __ldg(p.lengths + b);
       const float rbias = (p.row_bias && valid) ? __ldg(p.row_bias + (long long)b * p.T + t) : 0.f;
       const float* ub = (p.utt_bias && valid) ? p.utt_bias + (long long)b * p.ld_utt + n0 + half * 16 : nullptr;
       // stage this tile's per-column parameters (double-buffered by accumulator stage; the
@@ -517,6 +527,12 @@ tdnn_gemm_bf16x3_kernel(const __grid_constant__ CUtensorMap map_a_hi, const __gr
             }
           }
           f[4 * g + 0] = x0; f[4 * g + 1] = x1; f[4 * g + 2] = x2; f[4 * g + 3] = x3;
+        }
+        if constexpr (kMask) {
+          if (masked) {
+#pragma unroll
+            for (int j = 0; j < 16; ++j) f[j] = 0.f;
+          }
         }
         const int n = n0 + ch * 32;
         if (p.store_mode == 2) {
@@ -713,6 +729,9 @@ tdnn_gemm_bf16x3_kernel(const __grid_constant__ CUtensorMap map_a_hi, const __gr
                 x0 = 1.f / (1.f + expf(-x0)); x1 = 1.f / (1.f + expf(-x1));
                 x2 = 1.f / (1.f + expf(-x2)); x3 = 1.f / (1.f + expf(-x3));
               }
+            }
+            if constexpr (kMask) {
+              if (masked) { x0 = 0.f; x1 = 0.f; x2 = 0.f; x3 = 0.f; }
             }
             __nv_bfloat16 h0, l0, h1, l1, h2, l2, h3, l3;
             split_bf16(x0, h0, l0); split_bf16(x1, h1, l1); split_bf16(x2, h2, l2); split_bf16(x3, h3, l3);
@@ -975,10 +994,10 @@ struct GemmPlan {
   int out_Tdim = 0;          // time extent of the fp32 output map (k_slices for split-K)
 };
 
-template <int BLOCK_N, int kCta, int kNSub, bool kPool, bool kHist>
+template <int BLOCK_N, int kCta, int kNSub, bool kPool, bool kHist, bool kMask>
 static int launch_inst(const GemmPlan& pl, const CUtensorMap& my_f32, cudaStream_t stream) {
   using Cfg = GemmCfg<BLOCK_N, kCta, kNSub>;
-  XVB_ENSURE_DYN_SMEM((tdnn_gemm_bf16x3_kernel<BLOCK_N, kCta, kNSub, kPool, kHist>), Cfg::kSmemBytes);
+  XVB_ENSURE_DYN_SMEM((tdnn_gemm_bf16x3_kernel<BLOCK_N, kCta, kNSub, kPool, kHist, kMask>), Cfg::kSmemBytes);
   cudaLaunchConfig_t cfg{};
   cfg.gridDim = dim3(pl.grid);
   cfg.blockDim = dim3(kNumThreads);
@@ -993,13 +1012,13 @@ static int launch_inst(const GemmPlan& pl, const CUtensorMap& my_f32, cudaStream
   attr[1].val.programmaticStreamSerializationAllowed = 1;
   cfg.attrs = attr;
   cfg.numAttrs = pl.pdl ? 2 : 1;
-  XVB_CUDA(cudaLaunchKernelEx(&cfg, tdnn_gemm_bf16x3_kernel<BLOCK_N, kCta, kNSub, kPool, kHist>, pl.ma_hi, pl.ma_lo, pl.ma2_hi,
+  XVB_CUDA(cudaLaunchKernelEx(&cfg, tdnn_gemm_bf16x3_kernel<BLOCK_N, kCta, kNSub, kPool, kHist, kMask>, pl.ma_hi, pl.ma_lo, pl.ma2_hi,
                               pl.ma2_lo, pl.mw_hi, pl.mw_lo, pl.my_hi, pl.my_lo, my_f32, pl.p));
   XVB_LAUNCH_CHECK();
   return XVB_OK;
 }
 
-template <int BLOCK_N, int kCta, int kNSub = 1, bool kPool = false, bool kHist = false>
+template <int BLOCK_N, int kCta, int kNSub = 1, bool kPool = false, bool kHist = false, bool kMask = false>
 static int prepare_gemm(GemmPlan& pl, const void* w_hi, const void* w_lo) {
   using Cfg = GemmCfg<BLOCK_N, kCta, kNSub>;
   TdnnGemmParams& p = pl.p;
@@ -1040,7 +1059,7 @@ static int prepare_gemm(GemmPlan& pl, const void* w_hi, const void* w_lo) {
   pl.grid = (p.num_tiles < units ? p.num_tiles : units) * kCta;
   static const int pdl = getenv("XVB_PDL") ? atoi(getenv("XVB_PDL")) : 1;
   pl.pdl = pdl;
-  pl.launch = &launch_inst<BLOCK_N, kCta, kNSub, kPool, kHist>;
+  pl.launch = &launch_inst<BLOCK_N, kCta, kNSub, kPool, kHist, kMask>;
   return XVB_OK;
 }
 
@@ -1136,6 +1155,7 @@ int xvb::gemm_plan_build(GemmPlan** out, const xvb_tdnn_args_t& a, const TrialHi
   p.y_hi = reinterpret_cast<__nv_bfloat16*>(a.y_hi);
   p.y_lo = reinterpret_cast<__nv_bfloat16*>(a.y_lo);
   p.ldy = a.ldy; p.y_f32 = a.y_f32; p.ldyf = a.ldyf;
+  p.lengths = th ? nullptr : a.lengths;   // the histogram mode has no frames
 
   p.k_slices = splitk_slices(a, th != nullptr, &p.kb_per_slice);
   if (p.k_slices > 1) {
@@ -1148,6 +1168,7 @@ int xvb::gemm_plan_build(GemmPlan** out, const xvb_tdnn_args_t& a, const TrialHi
     p.y_f32 = static_cast<float*>(scratch); p.ldyf = Cout;
     p.bias = nullptr; p.scale = nullptr; p.shift = nullptr; p.flags = 0;
     p.store_mode = 0;
+    p.lengths = nullptr;   // segment level: one row per utterance, nothing to mask
   }
 
   if ((rc = make_frame_map(&pl.ma_hi, a.x_hi, Cin, T, B, a.ldx, p.Tb, p.Bb, a.x_batch_stride))) return rc;
@@ -1166,9 +1187,10 @@ int xvb::gemm_plan_build(GemmPlan** out, const xvb_tdnn_args_t& a, const TrialHi
   const int mode = gemm_cta_mode();
   const void* w_hi = a.w_hi;
   const void* w_lo = a.w_lo;
-  auto dispatch = [&]() -> int {
+  auto dispatch = [&](auto mask_tag) -> int {
+    constexpr bool kM = decltype(mask_tag)::value;
     if (a.pool_partial)  // fused pooling always runs on the swapped CTA-pair kernel (any shape: TMA zero-fills)
-      return prepare_gemm<256, 2, 1, true>(pl, w_hi, w_lo);
+      return prepare_gemm<256, 2, 1, true, false, kM>(pl, w_hi, w_lo);
     if (th)              // the diagonal test of the symmetric mode assumes 256-row units x 256-column tiles
       return prepare_gemm<256, 2, 1, false, true>(pl, w_hi, w_lo);
     static const int force_bn = getenv("XVB_GEMM_BN") ? atoi(getenv("XVB_GEMM_BN")) : 0;  // tuning knobs
@@ -1176,17 +1198,17 @@ int xvb::gemm_plan_build(GemmPlan** out, const xvb_tdnn_args_t& a, const TrialHi
     // accumulator in TMEM); measured slower end to end (profiles/r01_gemm_experiments.md), so opt-in.
     static const int wide = getenv("XVB_GEMM_WIDE") ? atoi(getenv("XVB_GEMM_WIDE")) : 0;
     if (mode == 2 && wide && force_bn != 128 && Cout >= 512 && (m_tiles / 2) * ((Cout + 511) / 512) >= sms / 2)
-      return prepare_gemm<256, 2, 2>(pl, w_hi, w_lo);
+      return prepare_gemm<256, 2, 2, false, false, kM>(pl, w_hi, w_lo);
     if (mode == 2 && force_bn != 128 && Cout >= 256 && m_tiles * ((Cout + 255) / 256) >= sms)
-      return prepare_gemm<256, 2>(pl, w_hi, w_lo);
+      return prepare_gemm<256, 2, 1, false, false, kM>(pl, w_hi, w_lo);
     if (mode == 2 && Cout >= 128 && m_tiles * ((Cout + 127) / 128) >= sms)
-      return prepare_gemm<128, 2>(pl, w_hi, w_lo);
-    if (Cout >= 256 && m_tiles * ((Cout + 255) / 256) >= sms) return prepare_gemm<256, 1>(pl, w_hi, w_lo);
-    if (Cout >= 128 && m_tiles * ((Cout + 127) / 128) >= sms) return prepare_gemm<128, 1>(pl, w_hi, w_lo);
-    if (Cout >= 64 && m_tiles * ((Cout + 63) / 64) >= sms / 2) return prepare_gemm<64, 1>(pl, w_hi, w_lo);
-    return prepare_gemm<32, 1>(pl, w_hi, w_lo);
+      return prepare_gemm<128, 2, 1, false, false, kM>(pl, w_hi, w_lo);
+    if (Cout >= 256 && m_tiles * ((Cout + 255) / 256) >= sms) return prepare_gemm<256, 1, 1, false, false, kM>(pl, w_hi, w_lo);
+    if (Cout >= 128 && m_tiles * ((Cout + 127) / 128) >= sms) return prepare_gemm<128, 1, 1, false, false, kM>(pl, w_hi, w_lo);
+    if (Cout >= 64 && m_tiles * ((Cout + 63) / 64) >= sms / 2) return prepare_gemm<64, 1, 1, false, false, kM>(pl, w_hi, w_lo);
+    return prepare_gemm<32, 1, 1, false, false, kM>(pl, w_hi, w_lo);
   };
-  if ((rc = dispatch())) return rc;
+  if ((rc = p.lengths ? dispatch(std::true_type{}) : dispatch(std::false_type{}))) return rc;
   guard.p = nullptr;
   *out = plp;
   return XVB_OK;

@@ -4,7 +4,8 @@ pytorch/libs/nnet/framework.py (for_extract_embedding :12-55, TopVirtualNnet :61
 Contract kept (SURVEY section 8b): `Cls(inputs_dim, num_targets, **params)` with `init()`,
 `load_state_dict(strict=False)` on the reference's keys, `.cuda()/.cpu()/.eval()`,
 `extract_embedding(feats[T,F] float32 ndarray) -> 1-D CPU float32 tensor`, the `maxChunk`
-splitting rule.  What is new: `extract_embedding_batch()` for equal-length utterances."""
+splitting rule.  What is new: `extract_embedding_batch()` for equal-length utterances and
+`extract_embedding_ragged()` for a list of utterances of any lengths."""
 import numpy as np
 import torch
 
@@ -161,6 +162,54 @@ class TopVirtualNnet(torch.nn.Module):
                 raise ValueError("T > maxChunk: use extract_embedding() per utterance")
             x = x.to(self.device_for_extraction(), non_blocking=True).contiguous()
             return self.extractor().extract(x)
+
+    def extract_embedding_ragged(self, feats_list):
+        """Utterances of different lengths in one call: a list of (T_i, F) float32 arrays or tensors, 1 <= T_i <= maxChunk
+        -> (N, D) float32 CPU tensor in input order, each row what extract_embedding() gives for that utterance alone.
+        TDNN x-vector extractors run length-sorted ragged batches (xvb_extractor_extract_ragged_shard_host); extractors
+        without a ragged path group the utterances by exact length and call extract_embedding_batch() per group."""
+        arrays = []
+        for i, f in enumerate(feats_list):
+            a = f.detach().cpu().numpy() if isinstance(f, torch.Tensor) else np.asarray(f)
+            if a.dtype != np.float32:
+                raise TypeError("extract_embedding_ragged expects float32 features, utterance {} is {}".format(i, a.dtype))
+            if a.ndim != 2 or a.shape[0] < 1:
+                raise ValueError("utterance {}: expected a (T, F) matrix with T >= 1, got shape {}".format(i, a.shape))
+            if a.shape[0] > 10000:
+                raise ValueError("utterance {} has {} frames > maxChunk (10000): use extract_embedding() for it".format(i, a.shape[0]))
+            arrays.append(a)
+        if not arrays:
+            raise ValueError("extract_embedding_ragged: empty list")
+        dev = self.device_for_extraction()
+        ex = self.extractor()
+        if not hasattr(ex, "extract_ragged_shard_host"):
+            groups = {}
+            for i, a in enumerate(arrays):
+                groups.setdefault(a.shape[0], []).append(i)
+            out = None
+            for idx in groups.values():
+                emb = self.extract_embedding_batch(np.stack([arrays[i] for i in idx])).cpu()
+                if out is None:
+                    out = torch.empty(len(arrays), emb.shape[1], dtype=torch.float32)
+                out[torch.as_tensor(idx)] = emb
+            return out
+        offsets = np.zeros(len(arrays) + 1, dtype=np.int64)
+        np.cumsum([a.shape[0] for a in arrays], out=offsets[1:])
+        if any(a.shape[1] != ex.feat_dim for a in arrays):
+            raise ValueError("expected {}-dim features".format(ex.feat_dim))
+        host = ex.staging_buffer(int(offsets[-1]))
+        hv = host.numpy()
+        for a, o0, o1 in zip(arrays, offsets[:-1], offsets[1:]):
+            hv[o0:o1] = a
+        train_status = self.training
+        self.eval()
+        try:
+            with torch.cuda.device(dev):
+                emb = ex.extract_ragged_shard_host(host, offsets)
+        finally:
+            if train_status:
+                self.train()
+        return torch.from_numpy(emb)
 
 
 def build_tdnn_extractor(model, inputs_dim, frame_layers, stats, tdnn6, tdnn7, extracted_embedding):

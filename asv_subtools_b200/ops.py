@@ -120,9 +120,10 @@ def fused_pool_layer(x, w, cout, context, bias=None, bn_scale=None, bn_shift=Non
 
 
 def tdnn_affine_ex(x, w, cout, context, x2=None, bias=None, bn_scale=None, bn_shift=None, utt_bias=None, row_bias=None,
-                   relu=False, tanh=False, sigmoid=False, y=None, y_f32=None, pool_partial=None):
+                   relu=False, tanh=False, sigmoid=False, y=None, y_f32=None, pool_partial=None, lengths=None):
     """Full form of the tcgen05 layer (xvb_tdnn_affine_ex).  x / x2: SplitPlanes (B,T,*) (views
-    allowed); y: SplitPlanes to write (view allowed) and/or y_f32: fp32 (B,T,>=cout) tensor."""
+    allowed); y: SplitPlanes to write (view allowed) and/or y_f32: fp32 (B,T,>=cout) tensor.  lengths: (B,) int32
+    CUDA tensor of valid frames per utterance (ragged batch: rows t >= lengths[b] come out as exact zeros)."""
     b, t = x.hi.shape[0], x.hi.shape[1]
     a = TdnnArgs()
     a.x_hi, a.x_lo, a.ldx = x.hi.data_ptr(), x.lo.data_ptr(), x.ld
@@ -148,6 +149,8 @@ def tdnn_affine_ex(x, w, cout, context, x2=None, bias=None, bn_scale=None, bn_sh
         a.y_f32, a.ldyf = y_f32.data_ptr(), y_f32.stride(-2)
     if pool_partial is not None:
         a.pool_partial = pool_partial.data_ptr()
+    if lengths is not None:
+        a.lengths = _req(lengths, torch.int32, "lengths").data_ptr()
     a.B, a.T, a.Cin, a.Cout = b, t, x.channels, cout
     check(lib.xvb_tdnn_affine_ex(C.byref(a), _stream()), "xvb_tdnn_affine_ex")
 
@@ -500,6 +503,23 @@ def trial_histogram(enroll, enroll_spk, test, test_spk, lo, hi, nbins=2048, row_
     return out
 
 
+# ------------------------------------------------------------------ ragged batching policy (host only)
+def ragged_plan(offsets, batch=256, max_frames=0):
+    """xvb_ragged_plan: offsets (N+1,) -> (order (N,) int32, list of per-batch index arrays into order).  Stable sort by
+    length, then batches of <= batch utterances with B * round_up(max L, 32) <= max_frames (<= 0: 262144)."""
+    off = np.ascontiguousarray(np.asarray(offsets, dtype=np.int64))
+    n = off.size - 1
+    if off.ndim != 1 or n < 1:
+        raise ValueError("ragged_plan: need (N+1,) offsets with N >= 1")
+    order = np.empty(n, dtype=np.int32)
+    first = np.empty(n + 1, dtype=np.int64)
+    nb = C.c_int64()
+    check(lib.xvb_ragged_plan(off.ctypes.data_as(C.c_void_p), n, int(batch), int(max_frames), order.ctypes.data_as(C.c_void_p),
+                              first.ctypes.data_as(C.c_void_p), C.byref(nb)), "xvb_ragged_plan")
+    first = first[:nb.value + 1]
+    return order, [order[first[k]:first[k + 1]] for k in range(nb.value)]
+
+
 # ------------------------------------------------------------------ whole-model extractor
 class Extractor:
     """Owner of a native xvb_extractor_t (packed weights + workspace on the current device)."""
@@ -630,6 +650,55 @@ class Extractor:
         """Replicated-table form of the shard calls (parallel.PeerTable.attach): every batch's embeddings also go to
         `ntables` table copies at row0 + row; ntables = 0 turns it off."""
         check(lib.xvb_extractor_set_gather(self._h, pointers, int(ntables), int(row0), int(ld)), "xvb_extractor_set_gather")
+
+    def extract_ragged(self, feats, offsets):
+        """Ragged batch: feats (sum_T, F) fp32 CUDA, utterance b = rows offsets[b] .. offsets[b+1] (host ints, B+1)
+        -> (B, D) fp32 CUDA, asynchronous on the current stream."""
+        feats = _req(feats, torch.float32, "feats")
+        if feats.dim() != 2 or feats.shape[1] != self.feat_dim:
+            raise ValueError("expected (sum_T, {}) features, got {}".format(self.feat_dim, tuple(feats.shape)))
+        off = np.ascontiguousarray(np.asarray(offsets, dtype=np.int64))
+        if off.ndim != 1 or off.size < 2 or off[-1] > feats.shape[0] or off.max() > np.iinfo(np.int32).max:
+            raise ValueError("offsets must be (B+1,) row indices into feats")
+        off = off.astype(np.int32)
+        b = off.size - 1
+        emb = torch.empty(b, self.embed_dim, dtype=torch.float32, device=feats.device)
+        check(lib.xvb_extractor_extract_ragged(self._h, _ptr(feats), off.ctypes.data_as(C.c_void_p), b, _ptr(emb), _stream()),
+              "xvb_extractor_extract_ragged")
+        return emb
+
+    def extract_ragged_shard_host(self, feats, offsets, batch=256, max_frames=0):
+        """N utterances of any lengths in host memory: feats (sum_T, F) float32 (ndarray or CPU tensor; staged through
+        pinned memory unless it is a pinned tensor already), offsets (N+1,) -> (N, D) float32 ndarray in input order.
+        Batches as xvb_ragged_plan cuts them (max_frames <= 0: 262144 padded frames per batch)."""
+        if isinstance(feats, torch.Tensor) and feats.is_pinned() and feats.dtype == torch.float32 and feats.is_contiguous():
+            host = feats
+        else:
+            src = torch.as_tensor(np.ascontiguousarray(feats, dtype=np.float32))
+            if src.dim() != 2:
+                raise ValueError("expected (sum_T, {}) features, got {}".format(self.feat_dim, tuple(src.shape)))
+            host = self.staging_buffer(src.shape[0])
+            host.copy_(src)
+        if host.dim() != 2 or host.shape[1] != self.feat_dim:
+            raise ValueError("expected (sum_T, {}) features, got {}".format(self.feat_dim, tuple(host.shape)))
+        off = np.ascontiguousarray(np.asarray(offsets, dtype=np.int64))
+        if off.ndim != 1 or off.size < 2 or off[-1] > host.shape[0]:
+            raise ValueError("offsets must be (N+1,) row indices into feats")
+        n = off.size - 1
+        emb = np.empty((n, self.embed_dim), dtype=np.float32)
+        check(lib.xvb_extractor_extract_ragged_shard_host(self._h, C.c_void_p(host.data_ptr()), off.ctypes.data_as(C.c_void_p), n,
+                                                          int(batch), int(max_frames), emb.ctypes.data_as(C.c_void_p), _stream()),
+              "xvb_extractor_extract_ragged_shard_host")
+        return emb
+
+    def staging_buffer(self, rows):
+        """(rows, F) float32 pinned host tensor, a view of a grow-only buffer this extractor keeps: pinning is expensive,
+        so repeated ragged calls reuse it.  Valid until the next call that stages through it."""
+        buf = getattr(self, "_pinned", None)
+        if buf is None or buf.shape[0] < rows:
+            buf = torch.empty(max(int(rows), 1), self.feat_dim, dtype=torch.float32, pin_memory=True)
+            self._pinned = buf
+        return buf[:rows]
 
     def extract_host_into(self, feats_ptr, b, t, emb_ptr):
         check(lib.xvb_extractor_extract_host(self._h, C.c_void_p(feats_ptr), b, t, C.c_void_p(emb_ptr), _stream()),

@@ -13,6 +13,11 @@ splitDataByLength.sh-balanced jobs); utterances longer than maxChunk fall back t
 per-utterance `extract_embedding()` with the reference's chunk rule.  One `FV` vector is written per
 input key (bucket order).  `--shard i/n` keeps every n-th utterance (one process per GPU without
 pre-splitting the scp).
+
+`--ragged true` replaces the exact-length buckets: utterances are collected in a window of up to
+`max_pending_frames` frames, the window is extracted with ONE `extract_embedding_ragged()` call
+(length-sorted batches of mixed lengths, each utterance computed as if alone), and the vectors are
+written in input order.  Utterances longer than maxChunk keep the per-utterance chunk rule.
 """
 import argparse
 import os
@@ -77,8 +82,21 @@ class Batcher:
         self.buckets, self.pending = {}, 0
 
 
-def extract_stream(model, reader, writer, batch_size=256, shard=(0, 1), log=print):
-    """reader yields (key, (T,F) float32 ndarray); writer(key, 1-D float32 ndarray)."""
+def run_window(model, window, writer):
+    """One ragged call for the window's utterances up to maxChunk frames, the chunk rule for longer ones; vectors are
+    written in window (= input) order."""
+    short = [f for _, f in window if f.shape[0] <= MAX_CHUNK]
+    embs = iter(model.extract_embedding_ragged(short).numpy()) if short else iter(())
+    for key, feats in window:
+        writer(key, next(embs) if feats.shape[0] <= MAX_CHUNK else model.extract_embedding(feats).numpy())
+
+
+def extract_stream(model, reader, writer, batch_size=256, shard=(0, 1), log=print, ragged=False,
+                   max_pending_frames=4_000_000):
+    """reader yields (key, (T,F) float32 ndarray); writer(key, 1-D float32 ndarray).  ragged: windows of up to
+    max_pending_frames frames through extract_embedding_ragged(), written in input order."""
+    if ragged:
+        return _extract_stream_ragged(model, reader, writer, shard, log, max_pending_frames)
     batcher = Batcher(batch_size)
     count = 0
 
@@ -108,6 +126,26 @@ def extract_stream(model, reader, writer, batch_size=256, shard=(0, 1), log=prin
     return count
 
 
+def _extract_stream_ragged(model, reader, writer, shard, log, max_pending_frames):
+    window, frames, count = [], 0, 0
+    for i, (key, feats) in enumerate(reader):
+        if i % shard[1] != shard[0]:
+            continue
+        log("Process utterance for key {0}".format(key))
+        feats = np.ascontiguousarray(feats)
+        if feats.dtype != np.float32:
+            raise TypeError("features of {} are {}, the extractor takes float32 (FM/CM) matrices".format(key, feats.dtype))
+        count += 1
+        window.append((key, feats))
+        frames += feats.shape[0]
+        if frames >= max_pending_frames:
+            run_window(model, window, writer)
+            window, frames = [], 0
+    if window:
+        run_window(model, window, writer)
+    return count
+
+
 def main(argv=None):
     ap = argparse.ArgumentParser(description="Extract embeddings from a piece of feats.scp or pipeline (B200)")
     ap.add_argument("--nnet-config", type=str, default="")
@@ -117,6 +155,9 @@ def main(argv=None):
     ap.add_argument("--gpu-id", type=str, default="")
     ap.add_argument("--batch-size", type=int, default=256)
     ap.add_argument("--shard", type=str, default="0/1", help="i/n: keep utterances with index %% n == i")
+    ap.add_argument("--ragged", type=str, default="false", choices=["true", "false"],
+                    help="true: mixed-length batches (extract_embedding_ragged) over windows of utterances, vectors in input "
+                         "order; false: exact-length buckets")
     ap.add_argument("--blueprint-dir", type=str, default="",
                     help="take the blueprint of the same file name from this directory (asv_subtools_b200/model) instead of "
                          "the path stored in nnet.config, so a reference model dir is used as it is")
@@ -147,7 +188,8 @@ def main(argv=None):
         # native ark reader (csrc/ark_io.cpp): the reference's byte-at-a-time key loop is the wall at GPU rates
         with kaldi_io.open_or_fd(args.vectors_wspecifier, "wb") as w:
             extract_stream(model, kaldi_io.read_mat_ark_native(args.feats_rspecifier),
-                           lambda k, v: kaldi_io.write_vec_flt(w, v, key=k), batch_size=args.batch_size, shard=(i, n))
+                           lambda k, v: kaldi_io.write_vec_flt(w, v, key=k), batch_size=args.batch_size, shard=(i, n),
+                           ragged=args.ragged == "true")
     except BaseException as err:
         if not isinstance(err, KeyboardInterrupt):
             traceback.print_exc()

@@ -127,6 +127,13 @@ typedef struct xvb_tdnn_args {
    * frame matrix (ntaps = 1, Cin = taps*channels), so a [-2..2] layer over 80 channels streams 7
    * channel blocks of 64 instead of 5 x (64 + 16).  Requires x2_* == NULL. */
   int64_t x_batch_stride;
+  /* Ragged batch: (B) int32 on the device, utterance b has lengths[b] valid frames (1 <= lengths[b] <= T);
+   * NULL: all T frames are valid.  Rows t >= lengths[b] of the plane / fp32 outputs are stored as exact
+   * zeros, so the next layer's taps past the end read what F.pad (components.py:117) gives the
+   * reference's one-utterance-at-a-time extraction (extract_embeddings.py:73-83); with pool_partial the
+   * epilogue counts lengths[b] frames (merge with the extractor's ragged path).  Ignored by the
+   * segment-level (T == 1, split-K) layers. */
+  const int32_t* lengths;
 } xvb_tdnn_args_t;
 int xvb_tdnn_affine_ex(const xvb_tdnn_args_t* args, void* stream);
 /* Time blocking the fused-pooling epilogue will use for a (B, T) batch. */
@@ -418,6 +425,33 @@ int xvb_extractor_extract_shard(xvb_extractor_t* h, const float* feats, int64_t 
                                 void* stream);
 int xvb_extractor_extract_shard_host(xvb_extractor_t* h, const float* feats_host, int64_t N, int T, int batch,
                                      float* emb_host, void* stream);
+/* ---------------------------------------------------------------------------------------------
+ * Ragged batches: utterances of different lengths in one call.  The reference extracts one utterance at a time
+ * (pytorch/pipeline/onestep/extract_embeddings.py:73-83), every TdnnAffine zero-padding its own input
+ * (libs/nnet/components.py:117), and StatisticsPooling averages over that utterance's frames (pooling.py:58-67).
+ * A ragged batch reproduces this per utterance: utterance b (L_b >= 1 frames) is padded to Tq = round_up(max L, 32),
+ * frame-layer rows t >= L_b are stored as exact zeros, and pooling counts L_b frames.  TDNN x-vector extractors with
+ * fused pooling only (XVB_ESTATE if it is switched off or a gather table is set).
+ *   _extract_ragged : feats (offsets_host[B], feat_dim) fp32 on the device, utterance b = rows offsets_host[b] ..
+ *                     offsets_host[b+1]; emb (B, embed_dim) on the device; asynchronous on `stream` (the lengths are
+ *                     uploaded on it from a pinned staging buffer the extractor owns).
+ *   _ragged_shard_host : N utterances in host memory (pinned, so that the copies overlap), int64 offsets (N+1)
+ *                     into feats_host; batches as xvb_ragged_plan cuts them with max_frames (<= 0: 262144) through
+ *                     the pipeline of xvb_extractor_extract_shard_host; emb_host (N, embed_dim) in INPUT order,
+ *                     complete when the call returns.
+ * Launch plans are cached per (B, Tq); at most 64 ragged ones per extractor lane (then they are rebuilt). */
+int xvb_extractor_extract_ragged(xvb_extractor_t* h, const float* feats, const int32_t* offsets_host, int B, float* emb,
+                                 void* stream);
+int xvb_extractor_extract_ragged_shard_host(xvb_extractor_t* h, const float* feats_host, const int64_t* offsets_host,
+                                            int64_t N, int batch, int64_t max_frames, float* emb_host, void* stream);
+/* The batching policy of ragged shards, host only (no device needed): stable sort of the N utterances by length
+ * (offsets_host (N+1) int64), then consecutive batches of <= `batch` utterances with B * round_up(max L, 32) <=
+ * max_frames (<= 0: 262144); an utterance longer than that forms a batch of its own.  order_out (N): utterance index
+ * per sorted position; batch k is order_out[batch_first_out[k] .. batch_first_out[k+1]), batch_first_out needs N+1
+ * entries; *num_batches_out = number of batches.  Replaces the exact-length buckets of the batching CLIs. */
+int xvb_ragged_plan(const int64_t* offsets_host, int64_t N, int batch, int64_t max_frames, int32_t* order_out,
+                    int64_t* batch_first_out, int64_t* num_batches_out);
+
 /* ---------------------------------------------------------------------------------------------
  * The embedding table of BASELINE configs[3] on every GPU of a node without a collective after extraction
  * (SURVEY 8e; replaces the `cat xvector.*.scp` of extract_xvectors_for_pytorch.sh:147-151 and the NCCL all-gather
