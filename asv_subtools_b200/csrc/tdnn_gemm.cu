@@ -497,6 +497,9 @@ tdnn_gemm_bf16x3_kernel(const __grid_constant__ CUtensorMap map_a_hi, const __gr
       const uint32_t slab = smem_u32(slab_base);
       const float relu_floor = relu ? 0.f : -INFINITY;   // branch-free ReLU switch
       const bool extras = rbias != 0.f || ub != nullptr || act_tanh || act_sigmoid;
+      // TMA stores clip the last 16-byte group of a row as a whole, so in the tile holding column Cout the columns
+      // [Cout, round_up(Cout, 16 bytes)) are written too: store zeros there (the pad split_f32 leaves), never epi(0)
+      const bool n_tail = n0 + kTileN > p.Cout;
 
       auto process = [&](uint32_t (&v)[16], int ch) {
         const int pc = ch * 32 + half * 16;
@@ -533,6 +536,10 @@ tdnn_gemm_bf16x3_kernel(const __grid_constant__ CUtensorMap map_a_hi, const __gr
 #pragma unroll
             for (int j = 0; j < 16; ++j) f[j] = 0.f;
           }
+        }
+        if (n_tail) {
+#pragma unroll
+          for (int j = 0; j < 16; ++j) f[j] = n0 + pc + j < p.Cout ? f[j] : 0.f;
         }
         const int n = n0 + ch * 32;
         if (p.store_mode == 2) {
@@ -732,6 +739,11 @@ tdnn_gemm_bf16x3_kernel(const __grid_constant__ CUtensorMap map_a_hi, const __gr
             }
             if constexpr (kMask) {
               if (masked) { x0 = 0.f; x1 = 0.f; x2 = 0.f; x3 = 0.f; }
+            }
+            if (n_tail) {
+              const int c = n0 + pc + 4 * g;
+              x0 = c < p.Cout ? x0 : 0.f; x1 = c + 1 < p.Cout ? x1 : 0.f;
+              x2 = c + 2 < p.Cout ? x2 : 0.f; x3 = c + 3 < p.Cout ? x3 : 0.f;
             }
             __nv_bfloat16 h0, l0, h1, l1, h2, l2, h3, l3;
             split_bf16(x0, h0, l0); split_bf16(x1, h1, l1); split_bf16(x2, h2, l2); split_bf16(x3, h3, l3);

@@ -80,15 +80,16 @@ def test_simt_layer_vs_oracle(ops, B, T, Cin, Cout, context, relu):
 
 
 GEMM_CASES = [
-    # B, T, Cin, Cout, context, relu, f32-out   (M tiles / N tiles / K tails exercised)
+    # B, T, Cin, Cout, context, relu, f32-out   (M tiles / N tiles / K tails exercised).  These small shapes run the
+    # <32,1,1> and <64,1,1> instantiations only; test_gpu_gemm_variants.py reaches the others.
     (2, 50, 24, 512, [-2, -1, 0, 1, 2], True, False),   # tdnn1, 23->24-dim MFCC: partial K step
     (3, 37, 80, 512, [-2, -1, 0, 1, 2], True, False),   # tdnn1, 80-dim fbank: 64+16 channel blocks, ragged T
     (2, 40, 512, 512, [-2, 0, 2], True, False),         # tdnn2: masked taps dropped
     (1, 7, 512, 512, [-3, 0, 3], True, False),          # tdnn3: T < context span, padding dominates
     (5, 16, 512, 512, [0], True, False),                # tdnn4
-    (2, 33, 512, 1500, [0], True, True),                # tdnn5: N tail (1500 = 5*256+220), fp32 out
+    (2, 33, 512, 1500, [0], True, True),                # tdnn5 shape, fp32 out: <32,1,1>, N tail 1500 = 46*32+28
     (9, 1, 3000, 512, [0], False, True),                # tdnn6.affine: segment level, M=B rows, narrow N tiles
-    (200, 8, 128, 128, [-2, 0, 2], True, False),        # Res2Net-shaped block, >148 tiles -> persistent loop
+    (200, 8, 128, 128, [-2, 0, 2], True, False),        # Res2Net-shaped block: 13 M blocks, 52 <32,1,1> tiles, one per CTA
     (16, 200, 512, 512, [-2, 0, 2], True, False),       # Tb=8 x Bb=16 tiling of the BASELINE shape
 ]
 
